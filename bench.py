@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- training-step throughput of the rasterizer hot path (BASELINE.json metric).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c2]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c2] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch of synthetic input: activations -> preprocess ->
 (all-to-all) -> tile binning + sort -> alpha blend -> fused L1+SSIM -> backward of all of it
@@ -44,7 +44,16 @@ def parse():
     ap.add_argument("--time-optimizer", action="store_true",
                     help="also time the fused Adam step (gs_adam_step) on the rank's parameters, reported separately under "
                          "'optimizer' (the headline metric excludes the optimizer, SURVEY.md 8d)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step computed as DIR/<name>.npy: the loss, the "
+                         "gradients of the six parameters, the screen-space gradient and the radii of a fixed, seeded "
+                         "sample of Gaussians (compare two builds output for output)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
+    return args
 
 
 def workload(args):
@@ -149,7 +158,6 @@ def cpu_arm(cfg, sample_n, steps, warmup):
     cam = syn.make_camera(W, H)
     sc = syn.make_scene(n, W, H, seed=0)
     gt = syn.make_gt_image(W, H)
-    steps, warmup = max(3, steps), max(2, warmup)
     for _ in range(warmup):
         out = o.train_step(sc, cam, gt)
     ts = []
@@ -174,7 +182,7 @@ def run_reference(args):
     if rank != 0:
         return
     cfg = workload(args)
-    steps, warmup = max(3, min(args.steps, 5)), max(2, min(args.warmup, 2))
+    steps, warmup = args.steps, 2
     r = cpu_arm(cfg, args.cpu_sample, steps, warmup)
     line = {"impl": "reference", "metric": METRIC, "value": r["value"], "unit": UNIT, "n_gpus": args.gpus,
             "steps": steps, "warmup": warmup, "ms_per_step": r["ms_per_step"], "higher_is_better": True,
@@ -226,6 +234,43 @@ def timed_steps(trainer, steps, resident, barrier_sync):
     barrier_sync()
     per = [evs[i].elapsed_time(evs[i + 1]) for i in range(steps)]
     return evs[0].elapsed_time(evs[steps]), per, out
+
+
+def dump_outputs(trainer, loss, out_dir, n_total, rank, world, dev):
+    """Writes what the last step of `trainer` computed, as a caller of Trainer.step receives it, to out_dir/<name>.npy:
+    the loss, the gradients of the six raw parameters, and per view the screen-space gradient (means2D.grad, which
+    densification reads) and the radii, all of one fixed, seeded sample of the Gaussians.  Each rank contributes the
+    sampled rows of its contiguous shard and rank 0 writes them in order, so the files have the same rows and layout for
+    any number of GPUs.  The sample keeps the files under 64 MB."""
+    import torch
+    import torch.distributed as dist
+    p = trainer.params
+    B = len(trainer.dcams)
+    rows = min(n_total, 1 << 16, (60 << 20) // (4 * (59 + 3 * B)))   # 59 parameter floats per Gaussian, 3 per view
+    sample = np.sort(np.random.default_rng(0).choice(n_total, size=rows, replace=False))
+    lo = n_total * rank // world
+    local = torch.from_numpy(sample[(sample >= lo) & (sample < lo + trainer.n_local)] - lo).to(dev)
+    m2 = trainer.means2D
+    m2_grad = torch.stack([t.grad for t in m2]) if isinstance(m2, list) else m2.grad
+    part = {f"grad{name}": getattr(p, name).grad[local] for name in
+            ("_xyz", "_features_dc", "_features_rest", "_scaling", "_rotation", "_opacity")}
+    part["grad_means2D"] = m2_grad[:, local]
+    part["radii"] = trainer._radii_local[:, local].float()
+    part = {k: v.float().cpu().numpy() for k, v in part.items()}
+    total = torch.tensor([loss], dtype=torch.float64, device=dev)
+    parts = [part]
+    if world > 1:
+        dist.all_reduce(total)                     # every rank's loss covers its own strips
+        parts = [None] * world
+        dist.all_gather_object(parts, part)
+    if rank != 0:
+        return
+    out = {k: np.concatenate([q[k] for q in parts], axis=1 if k in ("grad_means2D", "radii") else 0) for k in part}
+    out["loss"] = np.array(float(total.item()), np.float64)
+    out["sample_rows"] = sample.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in out.items():
+        np.save(os.path.join(out_dir, f"{k}.npy"), v)
 
 
 def run_ours(args):
@@ -296,6 +341,8 @@ def run_ours(args):
     ms2, per_step_e2e, loss_host = timed_steps(trainer, steps, False, barrier_sync)
     ms_e2e = max_over_ranks(ms2) / steps
     h2d, d2h = trainer.io_bytes_per_step()
+    if args.dump_outputs:   # before anything below runs another step or moves the parameters
+        dump_outputs(trainer, loss_host, args.dump_outputs, N, rank, world, dev)
 
     # ---- optional: the fused Adam step on this rank's six parameter tensors, after both timed regions ------------
     optimizer = None

@@ -1,56 +1,52 @@
-"""Drop-in smoke (SURVEY.md section 4 (v)): the REFERENCE's own modules import against our
-`diff_gaussian_rasterization` package, unchanged.  Needs /root/reference (authoring container only); skipped on the
-GPU box.  Nothing is executed on a device: the reference hard-codes "cuda" everywhere (SURVEY F3)."""
+"""Drop-in surface (SURVEY.md section 4 (v)): every name the reference's own modules reach in `diff_gaussian_rasterization`,
+`simple_knn._C`, `plyfile` and `gsplat`, the keywords it builds GaussianRasterizationSettings with and calls the operator
+with, and the tile grid it derives from get_block_XY() -- recorded from the reference by
+tests/golden/make_dropin_golden.py into tests/golden/dropin.json -- resolve against our packages, unchanged.  Nothing is
+executed on a device: the reference hard-codes "cuda" everywhere (SURVEY F3)."""
 import importlib
+import importlib.util
+import inspect
+import json
 import os
-import subprocess
-import sys
 
-import pytest
+G = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+PKG = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "grendel-gs_b200")
 
-REF = "/root/reference"
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
-pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "gaussian_renderer")), reason="reference not present")
-
-CODE = r"""
-import sys
-sys.path[:0] = [%(pkg)r, %(shims)r, %(ref)r]
-import diff_gaussian_rasterization as dgr
-assert dgr.__file__.startswith(%(pkg)r), dgr.__file__
-import arguments                               # arguments/__init__.py:17 imports the extension
-import gaussian_renderer                       # gaussian_renderer/__init__.py:14-25 (+ gsplat shim)
-import gaussian_renderer.workload_division as wd
-import gaussian_renderer.loss_distribution as ld
-import scene.gaussian_model                    # simple_knn._C.distCUDA2 + plyfile shims
-import utils.general_utils as utils
-assert gaussian_renderer.GaussianRasterizer is dgr.GaussianRasterizer
-assert gaussian_renderer.GaussianRasterizationSettings is dgr.GaussianRasterizationSettings
-assert wd.diff_gaussian_rasterization._C.get_local2j_ids_bool is dgr._C.get_local2j_ids_bool
-assert ld.diff_gaussian_rasterization.load_image_tiles_by_pos is dgr.load_image_tiles_by_pos
-# arguments/__init__.py:254-257: the block sizes come from the extension
-bx, by, one = dgr._C.get_block_XY()
-utils.set_block_size(bx, by, one)
-utils.set_img_size(1080, 1920)
-assert (utils.BLOCK_X, utils.BLOCK_Y, utils.ONE_DIM_BLOCK_SIZE, utils.TILE_Y, utils.TILE_X) == (16, 16, 256, 68, 120)
-# the settings object is built with exactly these keywords at gaussian_renderer/__init__.py:930-943
-import inspect, re
-src = inspect.getsource(gaussian_renderer.distributed_preprocess3dgs_and_all2all_final)
-kw = re.findall(r"^\s+(\w+)=", src[src.index("GaussianRasterizationSettings("):src.index("rasterizer = GaussianRasterizer")], flags=re.M)
-assert tuple(kw) == dgr.GaussianRasterizationSettings._fields, kw
-# and the operator is called with exactly these keywords (:949-956, :1271-1282)
-sig_p = inspect.signature(dgr.GaussianRasterizer.preprocess_gaussians).parameters
-for name in ("means3D", "scales", "rotations", "shs", "opacities", "cuda_args"):
-    assert name in sig_p, name
-sig_r = inspect.signature(dgr.GaussianRasterizer.render_gaussians).parameters
-for name in ("means2D", "conic_opacity", "rgb", "depths", "radii", "compute_locally", "extended_compute_locally", "cuda_args"):
-    assert name in sig_r, name
-print("DROPIN-IMPORTS-OK")
-"""
+def _shim(name, path):
+    """The opt-in stand-ins under shims/, loaded from their files so they cannot shadow a real install."""
+    spec = importlib.util.spec_from_file_location(f"{name}_shim", os.path.join(PKG, "shims", *path))
+    mod = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(mod)
+    return mod
 
 
 def test_reference_modules_import_against_our_package():
-    code = CODE % dict(pkg=os.path.join(ROOT, "grendel-gs_b200"), shims=os.path.join(ROOT, "grendel-gs_b200", "shims"), ref=REF)
-    r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=300, cwd="/tmp")
-    assert r.returncode == 0, r.stderr[-3000:]
-    assert "DROPIN-IMPORTS-OK" in r.stdout
+    rec = json.load(open(os.path.join(G, "dropin.json")))
+    import diff_gaussian_rasterization as dgr
+    from gs_b200 import ops
+    assert dgr.__file__.startswith(PKG), dgr.__file__
+    modules = {"diff_gaussian_rasterization": dgr, "simple_knn._C": importlib.import_module("simple_knn._C"),
+               "plyfile": _shim("plyfile", ("plyfile.py",)), "gsplat": _shim("gsplat", ("gsplat", "__init__.py"))}
+    assert set(rec["names_used"]) == set(modules)
+    for mod, names in rec["names_used"].items():
+        assert names, mod
+        for dotted in names:
+            obj = modules[mod]
+            for part in dotted.split("."):
+                assert hasattr(obj, part), f"{mod}.{dotted}"
+                obj = getattr(obj, part)
+    # arguments/__init__.py:254-257: the block sizes come from the extension, the reference derives its tile grid from them
+    g = rec["grid_1080p"]
+    assert dgr._C.get_block_XY() == (g["BLOCK_X"], g["BLOCK_Y"], g["ONE_DIM_BLOCK_SIZE"])
+    rs_1080p = dgr.GaussianRasterizationSettings(1080, 1920, 1.0, 1.0, None, 1.0, None, None, 3, None, False, False)
+    assert ops._tiles(rs_1080p) == (g["TILE_Y"], g["TILE_X"])
+    # the settings object is built with exactly these keywords at gaussian_renderer/__init__.py:930-943
+    assert tuple(rec["settings_keywords"]) == dgr.GaussianRasterizationSettings._fields, rec["settings_keywords"]
+    # and the operator is called with exactly these keywords (:949-956, :1271-1282)
+    sig_p = inspect.signature(dgr.GaussianRasterizer.preprocess_gaussians).parameters
+    for name in rec["preprocess_keywords"]:
+        assert name in sig_p, name
+    sig_r = inspect.signature(dgr.GaussianRasterizer.render_gaussians).parameters
+    for name in rec["render_keywords"]:
+        assert name in sig_r, name
