@@ -27,7 +27,8 @@
 //     just (T, behind-colour B): lanes that skip a splat run the same instructions with alpha = 0, which makes
 //     every update a no-op, so the blend path has no per-lane branches or conditional moves.
 //
-// Round 2: SEGMENT-PARALLEL backward (k_blend_bwd_seg, the default).  The forward stores, for every pixel of a tile, a
+// Round 2: SEGMENT-PARALLEL backward (k_blend_bwd_seg; round 3's default k_blend_bwd_seg3 walks the same way).  The
+// forward stores, for every pixel of a tile, a
 // checkpoint (T, colour summed over the LATER segments) every SEG_K entries of the tile list, so every (tile, SEG_K-entry
 // segment) can be walked back to front on its own.  One WARP owns one such unit and ALL 256 pixels of the tile: lane l
 // holds pixel l of each of the eight 8x4 blocks (state T and S = sum of the colour behind, weighted with dL/dpixel, in
@@ -356,6 +357,7 @@ GS_D p2 p2_add(p2 a, p2 b) { p2 r; asm("add.rn.f32x2 %0, %1, %2;" : "=l"(r) : "l
 // (separate result registers made ptxas copy every packed state variable back at the end of each iteration)
 GS_D void p2_fma_acc(p2 &c, p2 a, p2 b) { asm("fma.rn.f32x2 %0, %1, %2, %0;" : "+l"(c) : "l"(a), "l"(b)); }
 GS_D void p2_mul_acc(p2 &t, p2 f) { asm("mul.rn.f32x2 %0, %0, %1;" : "+l"(t) : "l"(f)); }
+GS_D void p2_add_acc(p2 &c, p2 a) { asm("add.rn.f32x2 %0, %0, %1;" : "+l"(c) : "l"(a)); }
 
 template <bool STATS, bool CKPT>
 __global__ void __launch_bounds__(F2_THREADS, F2_MIN_CTAS)
@@ -751,7 +753,7 @@ k_blend_bwd(int W, int H, int tiles_per_view, const float4 *__restrict__ rec, co
 }
 
 
-// ---- backward, segment-parallel (default) ------------------------------------------------------------------------
+// ---- backward, segment-parallel (round 2; kept behind gs_debug_set(GS_DEBUG_BWD_SEG_R2)) ----------------------------
 // One warp = one (tile, segment) unit, all 256 pixels of the tile: lane l owns pixel (l & 7, l >> 3) of each 8x4 block.
 // Per-pixel state, walking back to front:  T = transmittance in front of the current splat,
 //   S = sum over the entries BEHIND it of alpha_j T_j (c_j . dL/dpixel)  +  T_final (bg . dL/dpixel)
@@ -938,6 +940,265 @@ k_blend_bwd_seg(int W, int H, int tiles_per_view, const float4 *__restrict__ rec
     }
 }
 
+// ---- backward, segment-parallel, round 3 (default) ---------------------------------------------------------------------
+// The unit, the per-pixel state and the per-pixel arithmetic of k_blend_bwd_seg (which stays behind GS_DEBUG_BWD_SEG_R2 for
+// A/B runs); the nine sums of a splat hold the same values bit for bit, only their reduction over the warp is ordered
+// differently.  Fewer issued instructions per (splat, tile):
+//   * staging compacts a pass: only entries whose trimmed 8x4 mask is non-empty get a slot (and have their record
+//     gathered), so the walk spends nothing on an entry no block of the warp can use;
+//   * the sums accumulate as packed pairs (FMUL2 / FADD2 / FFMA2): (m dx, m dy), (m dx^2, m dx dy), colour 0 and 1;
+//   * two consecutive splats share the end of the reduction.  Each runs butterfly levels 16 and 8 on its own (down to 3
+//     values per lane: warp_reduce9_to3); the first one's 3 values wait in registers for the second, and levels 4, 2, 1
+//     reduce the 6 values of both at once (warp_reduce_pair: 22 instead of 28 shuffles per two splats), ending in ONE RED
+//     set of 18 lanes.  A splat left over at the end of the unit is reduced against zeros.
+
+// levels 16 and 8 of warp_reduce9: afterwards v[0] / v[1] hold value (lane >> 2 & 6) / (lane >> 2 & 6) + 1 summed over the
+// lanes that differ in bits 3 and 4, v[8] value 8 likewise
+GS_D void warp_reduce9_to3(float v[9], int lane) {
+    {
+        const bool h = lane & 16;
+#pragma unroll
+        for (int i = 0; i < 4; i++) {
+            const float send = h ? v[i] : v[i + 4], keep = h ? v[i + 4] : v[i];
+            v[i] = keep + __shfl_xor_sync(FULL, send, 16);
+        }
+    }
+    {
+        const bool h = lane & 8;
+#pragma unroll
+        for (int i = 0; i < 2; i++) {
+            const float send = h ? v[i] : v[i + 2], keep = h ? v[i + 2] : v[i];
+            v[i] = keep + __shfl_xor_sync(FULL, send, 8);
+        }
+    }
+    v[8] += __shfl_xor_sync(FULL, v[8], 16);
+    v[8] += __shfl_xor_sync(FULL, v[8], 8);
+}
+
+// levels 4, 2, 1 for two splats A and B (their warp_reduce9_to3 results).  Returns, in lane 4i the warp total of A's value i,
+// in lane 4i + 2 that of B's value i (i < 8), in lane 1 A's value 8 and in lane 5 B's value 8.
+GS_D float warp_reduce_pair(float a0, float a1, float a8, float b0, float b1, float b8, int lane) {
+    const bool h2 = lane & 4, h1 = lane & 2, h0 = lane & 1;
+    const float x = (h2 ? a1 : a0) + __shfl_xor_sync(FULL, h2 ? a0 : a1, 4);
+    const float y = (h2 ? b1 : b0) + __shfl_xor_sync(FULL, h2 ? b0 : b1, 4);
+    float z = (h2 ? b8 : a8) + __shfl_xor_sync(FULL, h2 ? a8 : b8, 4);
+    const float w = (h1 ? y : x) + __shfl_xor_sync(FULL, h1 ? x : y, 2);
+    z += __shfl_xor_sync(FULL, z, 2);
+    return (h0 ? z : w) + __shfl_xor_sync(FULL, h0 ? w : z, 1);
+}
+
+// the RED of warp_reduce_pair's result: role z = (row stride) | (splat B ? 256 : 0); only_a: the unit's last splat has no
+// partner
+GS_D void seg_red_pair(const uint4 ro, float val, uint32_t id_a, uint32_t id_b, bool only_a) {
+    float *rptr = reinterpret_cast<float *>((unsigned long long)ro.x | ((unsigned long long)ro.y << 32));
+    const bool second = ro.z & 256u;
+    const uint32_t id = second ? id_b : id_a;
+    // red.global: see k_blend_bwd_seg
+    if (rptr && !(only_a && second))
+        asm volatile("red.global.add.f32 [%0], %1;" ::"l"(rptr + (size_t)id * (ro.z & 255u)), "f"(val * __uint_as_float(ro.w))
+                     : "memory");
+}
+
+struct SegWarp3 {
+    SRec rec[SG_STAGE];      // compacted; c = (green, blue, 1 / opacity, splat id bits)
+    float4 pix[8 * 32];      // per pixel: dL/dpixel (3) and the number of live entries (int bits)
+    uint32_t mask[SG_STAGE]; // compacted: 8x4 block mask | (entry - pass start) << 8
+    uint4 role[32];          // per lane: RED target pointer (lo, hi), row stride | splat B, scale bits
+    float4 pend[32];         // per lane: the waiting splat's three partial sums and its id bits
+    SegCold cold;
+};
+
+__global__ void __launch_bounds__(SG_THREADS, SG_MIN_CTAS)
+k_blend_bwd_seg3(int W, int H, int tiles_per_view, const float4 *__restrict__ rec, const float *__restrict__ bg,
+                 const uint2 *__restrict__ ranges, const uint32_t *__restrict__ ids, const float *__restrict__ final_T,
+                 const uint32_t *__restrict__ n_contrib, const float *__restrict__ dL_dimage, const SegWs seg,
+                 float *__restrict__ d_means2D, float *__restrict__ d_conic_opacity, float *__restrict__ d_rgb) {
+    // one struct per warp, so that every per-lane slot is one base register plus a constant offset
+    __shared__ SegWarp3 s_all[SG_WARPS];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const uint32_t u = blockIdx.x * SG_WARPS + warp;
+    if (u >= *seg.n_units) return;  // warps are independent: no CTA-level synchronisation anywhere below
+    SegWarp3 &sw = s_all[warp];
+    SRec *s_rec = sw.rec;
+    float4 *s_pix = sw.pix + lane;
+    uint32_t *s_mask = sw.mask;
+    const uint2 unit = seg.units[u];
+    const int tile_g = (int)unit.x, sidx = (int)unit.y;
+    const int view = tile_g / tiles_per_view, tile = tile_g - view * tiles_per_view;
+    const int gx = (W + GS_BLOCK_X - 1) / GS_BLOCK_X;
+    const uint2 range = ranges[tile_g];
+    const int tl = (int)seg.tile_last[tile_g];
+    const int seg_base = sidx * SEG_K;
+    const int cnt = min(SEG_K, tl - seg_base);
+    const size_t HW = (size_t)H * W;
+    final_T += (size_t)view * HW;
+    n_contrib += (size_t)view * HW;
+    dL_dimage += (size_t)view * 3 * HW;
+    const int X0 = (tile % gx) * GS_BLOCK_X, Y0 = (tile / gx) * GS_BLOCK_Y;
+    const float bg0 = bg[0], bg1 = bg[1], bg2 = bg[2];
+    const float4 *ck = seg.ckpt + ((size_t)(range.x / SEG_K) + tile_g + sidx) * SEG_SLOT + lane;
+    float T[8], S[8];
+    uint32_t blive = 0, blive_hi = 0;  // byte b: deepest live entry of block b over the warp
+#pragma unroll
+    for (int b = 0; b < 8; b++) {
+        const int px = X0 + (b & 1) * 8 + (lane & 7), py = Y0 + (b >> 1) * 4 + (lane >> 3);
+        const bool inside = px < W && py < H;
+        const size_t pix = (size_t)py * W + px;
+        float Tf = 0.f, d0 = 0.f, d1 = 0.f, d2 = 0.f;
+        int last = 0;
+        if (inside) {
+            Tf = final_T[pix];
+            last = (int)n_contrib[pix];
+            d0 = dL_dimage[pix]; d1 = dL_dimage[HW + pix]; d2 = dL_dimage[2 * HW + pix];
+        }
+        const float sbg = Tf * (bg0 * d0 + bg1 * d1 + bg2 * d2);
+        T[b] = Tf;
+        S[b] = sbg;
+        if (last > seg_base + SEG_K) {  // alive beyond this segment: the forward left its state at the boundary
+            const float4 c = ck[b * 32];
+            T[b] = c.x;
+            S[b] = c.y * d0 + c.z * d1 + c.w * d2 + sbg;
+        }
+        const int live = max(0, min(SEG_K, last - seg_base));  // entries [0, live) of the segment are in front of the
+        s_pix[b * 32] = make_float4(d0, d1, d2, __int_as_float(live));  // pixel's last contributor
+        const uint32_t m = __reduce_max_sync(FULL, (uint32_t)live);
+        if (b < 4) blive |= m << (8 * b); else blive_hi |= m << (8 * (b - 4));
+    }
+    {   // lane roles of the final RED (warp_reduce_pair): lane 4i / 4i + 2 add value i of splat A / B, lane 1 / 5 value 8
+        const bool even = !(lane & 1);
+        const int role = even ? (lane >> 2) : (lane == 1 || lane == 5 ? 8 : -1);
+        const uint32_t second = even ? (lane >> 1) & 1 : (lane >> 2) & 1;
+        float *rptr = nullptr;
+        uint32_t rstride = 0;
+        float rscale = 0.f;
+        if (role >= 0) {
+            if (role < 2) { rptr = d_means2D + role; rstride = 2; rscale = role == 0 ? -0.5f * (float)W : -0.5f * (float)H; }
+            else if (role < 6) { rptr = d_conic_opacity + (role - 2); rstride = 4; rscale = role == 3 ? -1.f : (role == 5 ? 1.f : -0.5f); }
+            else { rptr = d_rgb + (role - 6); rstride = 3; rscale = 1.f; }
+        }
+        const unsigned long long rp = (unsigned long long)rptr;
+        sw.role[lane] = make_uint4((uint32_t)rp, (uint32_t)(rp >> 32), rstride | (second << 8), __float_as_uint(rscale));
+        if (lane == 0) {
+            SegCold c;
+            c.ids = ids + range.x + seg_base; c.cull = seg.cull + range.x + seg_base; c.cnt = cnt; c.blive = blive; c.blive_hi = blive_hi;
+            sw.cold = c;
+        }
+    }
+    const uint4 *s_role = &sw.role[lane];
+    const SegCold *s_cold = &sw.cold;
+    const float pxf0 = (float)(X0 + (lane & 7)), pyf0 = (float)(Y0 + (lane >> 3));
+    // a splat waiting for a partner in the shared reduction tail keeps its three partial sums and its id in shared memory
+    // (in registers they pushed the walk's state into local memory)
+    float4 *s_pend = &sw.pend[lane];
+    bool pend = false;
+    for (int p0 = (cnt - 1) & ~(SG_STAGE - 1); p0 >= 0; p0 -= SG_STAGE) {
+        // stage up to 32 entries, one per lane; entry i keeps only the blocks it can reach that still have a live pixel at
+        // depth i, and only entries with a block left get a (compacted) slot
+        __syncwarp();
+        const SegCold cold = *s_cold;
+        const int pn = min(SG_STAGE, cold.cnt - p0);
+        uint32_t m = 0u;
+        if (lane < pn) {
+            const int i = p0 + lane;
+            // the forward's 4x4-block mask of this entry; an 8x4 block is two horizontally adjacent 4x4 blocks: OR the bit
+            // pairs, then pack the even bits
+            m = cold.cull[i];
+            m = (m | (m >> 1)) & 0x5555u;
+            m = (m | (m >> 1)) & 0x3333u;
+            m = (m | (m >> 2)) & 0x0f0fu;
+            m = (m | (m >> 4)) & 0x00ffu;
+#pragma unroll
+            for (int q = 0; q < 8; q++) {
+                const uint32_t bl = ((q < 4 ? cold.blive : cold.blive_hi) >> (8 * (q & 3))) & 0xffu;
+                if ((uint32_t)i >= bl) m &= ~(1u << q);
+            }
+        }
+        const uint32_t act = __ballot_sync(FULL, m != 0u);
+        if (m != 0u) {
+            const int slot = __popc(act & ((1u << lane) - 1u));
+            const uint32_t g = cold.ids[p0 + lane];
+            const float4 *r = rec + (size_t)3 * g;
+            const float4 a = __ldg(r), b = __ldg(r + 1), c = __ldg(r + 2);
+            // positive form q = -power, t = -thr (see k_blend_fwd2's staging): the pixel test is one unsigned compare
+            s_rec[slot].a = make_float4(a.x, a.y, -a.z, -a.w);
+            s_rec[slot].b = make_float4(-b.x, b.y, fmaxf(-b.z, 0.f), b.w);
+            s_rec[slot].c = make_float4(c.x, c.y, gs_rcp_approx(b.y), __uint_as_float(g));
+            s_mask[slot] = m | ((uint32_t)lane << 8);
+        }
+        __syncwarp();
+        for (int k = __popc(act) - 1; k >= 0; k--) {
+            // warp-uniform by construction; the redux makes that visible to the compiler (see k_blend_bwd_seg)
+            const uint32_t mw8 = __reduce_or_sync(FULL, s_mask[k]);
+            const uint32_t m8 = mw8 & 0xffu;
+            const int j = p0 + (int)(mw8 >> 8);
+            const float4 a = s_rec[k].a, b4 = s_rec[k].b;
+            const float2 c4 = *reinterpret_cast<const float2 *>(&s_rec[k].c);  // (green, blue)
+            const float mxl = a.x - pxf0, myl = a.y - pyf0;
+            // the nine sums: (m dx, m dy), (m dx^2, m dx dy), m dy^2, m, (colour 0, colour 1), colour 2
+            const p2 zero2 = p2_bc(0.f);
+            p2 s01 = zero2, s23 = zero2, s67 = zero2;
+            float s4 = 0.f, s5 = 0.f, s8 = 0.f;
+            bool any_full = false;
+#pragma unroll
+            for (int b = 0; b < 8; b++) {
+                if (m8 & (1u << b)) {
+                    const float4 pc = s_pix[b * 32];
+                    const float dx = mxl - (float)((b & 1) * 8), dy = myl - (float)((b >> 1) * 4);
+                    const float q = dx * (a.z * dx + a.w * dy) + b4.x * dy * dy;   // -power
+                    const bool ok = (j < __float_as_int(pc.w)) && __float_as_uint(q) <= __float_as_uint(b4.z);
+                    if (__any_sync(FULL, ok)) {
+                        const float G = gs_exp_neg(-q);
+                        const float alpha = fminf(ALPHA_MAX, b4.y * G);
+                        const float ae = ok ? alpha : 0.f;   // effective alpha: 0 = this lane skips the splat
+                        float inv;                            // 1/(1-ae), 1-ae in [0.01, 1]: one MUFU.RCP
+                        asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(inv) : "f"(1.f - ae));
+                        const float Tk = T[b] * inv;          // transmittance in front of this splat
+                        T[b] = Tk;
+                        const float cd = b4.w * pc.x + c4.x * pc.y + c4.y * pc.z;
+                        const float dL_dalpha = cd * Tk - S[b] * inv;
+                        const float mw = ok ? b4.y * dL_dalpha * G : 0.f;
+                        const float dch = ae * Tk;
+                        S[b] += dch * cd;
+                        const p2 d = p2_make(dx, dy);
+                        const p2 mxy = p2_mul(p2_bc(mw), d);                 // (m dx, m dy)
+                        p2_add_acc(s01, mxy);
+                        p2_fma_acc(s23, p2_bc(p2_lo(mxy)), d);               // (m dx dx, m dx dy)
+                        s4 += p2_hi(mxy) * dy;
+                        s5 += mw;
+                        p2_fma_acc(s67, p2_bc(dch), p2_make(pc.x, pc.y));
+                        s8 += dch * pc.z;
+                        any_full = true;
+                    }
+                }
+            }
+            if (!any_full) continue;
+            float v[9];
+            {   // per-lane pre-mix as in k_blend_bwd_seg: every reduced value is ONE output element
+                const float sx = p2_lo(s01), sy = p2_hi(s01);
+                v[0] = 2.f * a.z * sx + a.w * sy;
+                v[1] = 2.f * b4.x * sy + a.w * sx;
+                v[2] = p2_lo(s23); v[3] = p2_hi(s23); v[4] = s4;
+                v[5] = s5 * s_rec[k].c.z;
+                v[6] = p2_lo(s67); v[7] = p2_hi(s67); v[8] = s8;
+            }
+            warp_reduce9_to3(v, lane);
+            const uint32_t id = __float_as_uint(s_rec[k].c.w);
+            if (!pend) {
+                *s_pend = make_float4(v[0], v[1], v[8], __uint_as_float(id));
+                pend = true;
+                continue;
+            }
+            const float4 pa = *s_pend;
+            seg_red_pair(*s_role, warp_reduce_pair(pa.x, pa.y, pa.z, v[0], v[1], v[8], lane), __float_as_uint(pa.w), id, false);
+            pend = false;
+        }
+    }
+    if (pend) {
+        const float4 pa = *s_pend;
+        seg_red_pair(*s_role, warp_reduce_pair(pa.x, pa.y, pa.z, 0.f, 0.f, 0.f, lane), __float_as_uint(pa.w), 0u, true);
+    }
+}
+
 template <bool STATS, bool CKPT>
 static void launch_fwd(int grid, cudaStream_t stream, int W, int H, int T1, const float *rec, const float *bg,
                        const uint8_t *cl, const uint32_t *ranges, const uint32_t *ids, float *image, float *final_T,
@@ -1024,10 +1285,17 @@ extern "C" int gs_render_backward_batched(int num_views, int P, int64_t R, int i
         }
         const SegWs seg = seg_carve(const_cast<void *>(seg_ws), R, T);
         const int64_t max_units = R / SEG_K + T;   // >= sum over tiles of ceil(walked entries / SEG_K)
-        k_blend_bwd_seg<<<(unsigned)((max_units + SG_WARPS - 1) / SG_WARPS), SG_THREADS, 0, stream>>>(
-            image_width, image_height, gx * gy, reinterpret_cast<const float4 *>(rec), bg,
-            reinterpret_cast<const uint2 *>(ranges), ids_sorted, final_T, n_contrib, dL_dimage, seg, dL_dmeans2D,
-            dL_dconic_opacity, dL_drgb);
+        const unsigned grid = (unsigned)((max_units + SG_WARPS - 1) / SG_WARPS);
+        if (g_gs_debug_flags & GS_DEBUG_BWD_SEG_R2)
+            k_blend_bwd_seg<<<grid, SG_THREADS, 0, stream>>>(
+                image_width, image_height, gx * gy, reinterpret_cast<const float4 *>(rec), bg,
+                reinterpret_cast<const uint2 *>(ranges), ids_sorted, final_T, n_contrib, dL_dimage, seg, dL_dmeans2D,
+                dL_dconic_opacity, dL_drgb);
+        else
+            k_blend_bwd_seg3<<<grid, SG_THREADS, 0, stream>>>(
+                image_width, image_height, gx * gy, reinterpret_cast<const float4 *>(rec), bg,
+                reinterpret_cast<const uint2 *>(ranges), ids_sorted, final_T, n_contrib, dL_dimage, seg, dL_dmeans2D,
+                dL_dconic_opacity, dL_drgb);
         GS_LAUNCH_CHECK();
         return GS_OK;
     }

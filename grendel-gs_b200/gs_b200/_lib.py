@@ -140,6 +140,7 @@ DEBUG_NO_BLOCK_CULL = 1
 DEBUG_BWD_TILE = 2       # gs_render_backward: round 1's tile-parallel kernel instead of the segment-parallel one
 DEBUG_FWD_HALFWARP = 4   # gs_render_forward: round 1's half-warp blend kernel instead of the packed two-pixel one
 DEBUG_XR_PACK_CTA = 8    # direct exchange: CTA-compacted pack kernel (A/B switch)
+DEBUG_BWD_SEG_R2 = 16    # gs_render_backward: round 2's segment-parallel kernel instead of round 3's (A/B switch)
 
 
 def debug_set(flags):

@@ -273,7 +273,11 @@ enum {
     GS_DEBUG_FWD_HALFWARP = 4,
     /* direct exchange: pack with a CTA-level compaction per destination (one row per thread, 200-400-byte NVLink spans)
      * instead of per-warp stores; same rows, same bytes (A/B switch until it is measured at 8 ranks) */
-    GS_DEBUG_XR_PACK_CTA = 8
+    GS_DEBUG_XR_PACK_CTA = 8,
+    /* gs_render_backward with a segment workspace: round 2's segment-parallel kernel (k_blend_bwd_seg, one reduction and
+     * RED set per splat) instead of round 3's (k_blend_bwd_seg3: compacted passes, packed sums, reduction tail shared by
+     * two splats); the same sums, reduced in a different order.  GS_DEBUG_BWD_TILE takes precedence. */
+    GS_DEBUG_BWD_SEG_R2 = 16
 };
 GS_API int gs_debug_set(int flags);
 
