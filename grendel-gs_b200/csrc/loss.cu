@@ -10,6 +10,11 @@
 //
 // HBM bound: forward reads 15 B and writes 36 B per pixel-channel triple (three derivative maps kept for
 // the backward), backward reads 51 B and writes 12 B; no tensor-core shaped work.
+//
+// The same forward kernel, instantiated in a metrics mode (gs_metrics_batched), evaluates held-out views: per view and
+// channel the fp64 sums of |x - y|, (x - y)^2 and ssim_map(x, y) over the counted rows, with x = clamp(image, 0, 1)
+// (train_internal.py:471-478) or that image after the 8-bit PNG round trip of render.py:127-138 -> metrics.py:26-36.
+// It reads 15 B per pixel-channel triple and writes only the 9 sums per view.
 #include "common.cuh"
 
 #define LS_TILE 32
@@ -45,10 +50,31 @@ struct LossViews {
     unsigned long long map_off[GS_MAX_VIEWS];         // float offset of the view's 9 derivative planes in `maps`
 };
 
+// What k_loss_fwd computes from the rendered pixel x and the ground truth y = gt_u8 / 255.
+enum LossMode {
+    LS_LOSS = 0,            // training loss: x as rendered; sums[2 view + {0,1}] = sum |x-y|, sum ssim_map; derivative maps
+    LS_METRICS_REPORT = 1,  // x = clamp(x, 0, 1); sums[9 view + 3 q + c] (q = |x-y|, (x-y)^2, ssim_map; c = channel); no maps
+    LS_METRICS_SAVED = 2,   // as REPORT, x quantised to 8 bits the way torchvision.utils.save_image does, then read back
+};
+
+// The evaluated pixel value.  SAVED: save_image's mul(255).add_(0.5).clamp_(0, 255).to(uint8) with the multiply and the
+// add rounded separately (no FMA contraction), then to_tensor's division by 255.
+template <int MODE>
+__device__ __forceinline__ float metric_input(float v) {
+    v = fminf(1.f, fmaxf(0.f, v));
+    if (MODE == LS_METRICS_SAVED) {
+        const float q = fminf(255.f, fmaxf(0.f, __fadd_rn(__fmul_rn(v, 255.f), 0.5f)));
+        v = (float)(int)q / 255.0f;
+    }
+    return v;
+}
+
 // temp layout: [0,16) two double accumulators per view; then maps (3 maps x 3 channels x rows x W per view)
+template <int MODE>
 __global__ void __launch_bounds__(LS_THREADS)
 k_loss_fwd(int W, int H, const LossViews lv, const float *__restrict__ image, float *__restrict__ maps,
            double *__restrict__ sums) {
+    constexpr bool kMetrics = MODE != LS_LOSS;
     __shared__ float s_x[LS_IN][LS_IN + 1], s_y[LS_IN][LS_IN + 1];
     __shared__ float s_h[5][LS_IN][LS_TILE + 1];
     __shared__ float s_red[2][LS_THREADS / 32];
@@ -59,10 +85,18 @@ k_loss_fwd(int W, int H, const LossViews lv, const float *__restrict__ image, fl
     const size_t HW = (size_t)H * W, SW = (size_t)rows * W;
     const uint8_t *__restrict__ gt = lv.gt[view];
     image += (size_t)view * 3 * HW;
-    maps += lv.map_off[view];
-    sums += 2 * view;
+    if constexpr (kMetrics) {
+        sums += 9 * view;
+    } else {
+        maps += lv.map_off[view];
+        sums += 2 * view;
+    }
     const float C1 = 0.01f * 0.01f, C2 = 0.03f * 0.03f;
     float l1 = 0.f, ss = 0.f;
+    // metrics: every per-pixel term is added in fp64, so a view's sums do not depend on how its rows are split into
+    // windows and tiles beyond the order of fp64 additions
+    __shared__ double s_msum[3][3][LS_THREADS / 32];   // [quantity][channel][warp]; allocated only where it is used
+    double m_sad = 0.0, m_sse = 0.0, m_ssim = 0.0;
     for (int ch = 0; ch < 3; ch++) {
         for (int k = threadIdx.x; k < LS_IN * LS_IN; k += LS_THREADS) {
             const int r = k / LS_IN, c = k % LS_IN;
@@ -70,6 +104,7 @@ k_loss_fwd(int W, int H, const LossViews lv, const float *__restrict__ image, fl
             float vx = 0.f, vy = 0.f;
             if (y >= 0 && y < rows && x >= 0 && x < W) {
                 vx = image[ch * HW + (size_t)(row0 + y) * W + x];
+                if constexpr (kMetrics) vx = metric_input<MODE>(vx);
                 vy = fminf(1.f, fmaxf(0.f, (float)gt[ch * SW + (size_t)y * W + x] / 255.0f));
             }
             s_x[r][c] = vx; s_y[r][c] = vy;
@@ -115,7 +150,18 @@ k_loss_fwd(int W, int H, const LossViews lv, const float *__restrict__ image, fl
 #pragma unroll
             for (int q = 0; q < 4; q++) {
                 const int r = r0 + q, y = ty0 + r;
-                if (y < rows && x < W) {
+                if constexpr (kMetrics) {
+                    if (y < rows && x < W && y >= crow0 && y < crow1) {
+                        const float s1 = e11[q] - m1[q] * m1[q], s2 = e22[q] - m2[q] * m2[q], s12 = e12[q] - m1[q] * m2[q];
+                        const float A = 2.f * m1[q] * m2[q] + C1, B = 2.f * s12 + C2,
+                                    Cc = m1[q] * m1[q] + m2[q] * m2[q] + C1, D = s1 + s2 + C2;
+                        const float iCD = 1.f / (Cc * D);
+                        m_ssim += (double)(A * B * iCD);
+                        const float d = s_x[r + LS_HALO][c + LS_HALO] - s_y[r + LS_HALO][c + LS_HALO];
+                        m_sad += (double)fabsf(d);
+                        m_sse += (double)d * (double)d;
+                    }
+                } else if (y < rows && x < W) {
                     const size_t o = (size_t)ch * SW + (size_t)y * W + x;
                     if (y < crow0 || y >= crow1) {  // halo row: feeds the neighbours' windows, carries no loss itself
                         maps[o] = 0.f; maps[3 * SW + o] = 0.f; maps[6 * SW + o] = 0.f;
@@ -135,16 +181,38 @@ k_loss_fwd(int W, int H, const LossViews lv, const float *__restrict__ image, fl
                 }
             }
         }
+        if constexpr (kMetrics) {   // this channel's three sums: warp tree, then one slot per warp
+#pragma unroll
+            for (int o = 16; o > 0; o >>= 1) {
+                m_sad += __shfl_xor_sync(0xffffffffu, m_sad, o);
+                m_sse += __shfl_xor_sync(0xffffffffu, m_sse, o);
+                m_ssim += __shfl_xor_sync(0xffffffffu, m_ssim, o);
+            }
+            if ((threadIdx.x & 31) == 0) {
+                s_msum[0][ch][threadIdx.x >> 5] = m_sad; s_msum[1][ch][threadIdx.x >> 5] = m_sse;
+                s_msum[2][ch][threadIdx.x >> 5] = m_ssim;
+            }
+            m_sad = m_sse = m_ssim = 0.0;
+        }
         __syncthreads();
     }
+    if constexpr (kMetrics) {
+        if (threadIdx.x < 9) {
+            const int q = threadIdx.x / 3, c = threadIdx.x % 3;
+            double a = 0.0;
+            for (int w = 0; w < LS_THREADS / 32; w++) a += s_msum[q][c][w];
+            atomicAdd(&sums[3 * q + c], a);
+        }
+    } else {
 #pragma unroll
-    for (int o = 16; o > 0; o >>= 1) { l1 += __shfl_xor_sync(0xffffffffu, l1, o); ss += __shfl_xor_sync(0xffffffffu, ss, o); }
-    if ((threadIdx.x & 31) == 0) { s_red[0][threadIdx.x >> 5] = l1; s_red[1][threadIdx.x >> 5] = ss; }
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        double a = 0.0, b = 0.0;
-        for (int w = 0; w < LS_THREADS / 32; w++) { a += (double)s_red[0][w]; b += (double)s_red[1][w]; }
-        atomicAdd(&sums[0], a); atomicAdd(&sums[1], b);
+        for (int o = 16; o > 0; o >>= 1) { l1 += __shfl_xor_sync(0xffffffffu, l1, o); ss += __shfl_xor_sync(0xffffffffu, ss, o); }
+        if ((threadIdx.x & 31) == 0) { s_red[0][threadIdx.x >> 5] = l1; s_red[1][threadIdx.x >> 5] = ss; }
+        __syncthreads();
+        if (threadIdx.x == 0) {
+            double a = 0.0, b = 0.0;
+            for (int w = 0; w < LS_THREADS / 32; w++) { a += (double)s_red[0][w]; b += (double)s_red[1][w]; }
+            atomicAdd(&sums[0], a); atomicAdd(&sums[1], b);
+        }
     }
 }
 
@@ -283,7 +351,7 @@ static int loss_forward_impl(int num_views, int H, int W, const int32_t *rows4, 
     GsStageTimer timer(GS_STAGE_LOSS_FWD, stream);
     if (max_rows > 0) {
         dim3 grid((W + LS_TILE - 1) / LS_TILE, (max_rows + LS_TILE - 1) / LS_TILE, num_views);
-        k_loss_fwd<<<grid, LS_THREADS, 0, stream>>>(W, H, lv, image, maps, sums);
+        k_loss_fwd<LS_LOSS><<<grid, LS_THREADS, 0, stream>>>(W, H, lv, image, maps, sums);
         GS_LAUNCH_CHECK();
     }
     k_loss_finalize<<<1, 2 * GS_MAX_VIEWS, 0, stream>>>(num_views, sums, 1.0 / (3.0 * (double)H * (double)W), out);
@@ -367,4 +435,31 @@ extern "C" int gs_loss_backward_batched(int num_views, int image_height, int ima
                                         const float *grad_l1, const float *grad_ssim, float *dL_dimage, void *stream_) {
     return loss_backward_impl(num_views, image_height, image_width, rows4_host, image, gt_u8_ptrs_host, temp, grad_l1,
                               grad_ssim, dL_dimage, LS_HEADER_B, (cudaStream_t)stream_);
+}
+
+extern "C" int gs_metrics_batched(int num_views, int image_height, int image_width, const int32_t *rows4_host,
+                                  const float *images, const uint8_t *const *gt_u8_host_array, int saved_mode,
+                                  double *out_sums, void *stream_) {
+    GS_REQUIRE(images && out_sums, "null pointer");
+    GS_REQUIRE(saved_mode == 0 || saved_mode == 1, "saved_mode must be 0 or 1");
+    const cudaStream_t stream = (cudaStream_t)stream_;
+    LossViews lv;
+    int max_rows = 0;
+    size_t sum_rows = 0;
+    int rc = make_loss_views(num_views, image_height, image_width, rows4_host, (const void *const *)gt_u8_host_array, lv,
+                             &max_rows, &sum_rows);
+    if (rc != GS_OK) return rc;
+    rc = ensure_gauss();
+    if (rc != GS_OK) return rc;
+    GS_CUDA_TRY(cudaMemsetAsync(out_sums, 0, 9 * sizeof(double) * (size_t)num_views, stream));
+    if (max_rows == 0) return GS_OK;
+    dim3 grid((image_width + LS_TILE - 1) / LS_TILE, (max_rows + LS_TILE - 1) / LS_TILE, num_views);
+    if (saved_mode)
+        k_loss_fwd<LS_METRICS_SAVED><<<grid, LS_THREADS, 0, stream>>>(image_width, image_height, lv, images, nullptr,
+                                                                       out_sums);
+    else
+        k_loss_fwd<LS_METRICS_REPORT><<<grid, LS_THREADS, 0, stream>>>(image_width, image_height, lv, images, nullptr,
+                                                                        out_sums);
+    GS_LAUNCH_CHECK();
+    return GS_OK;
 }

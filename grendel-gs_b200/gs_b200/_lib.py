@@ -52,6 +52,7 @@ SIGNATURES = {
     "gs_loss_temp_bytes_batched": (_sz, [_i, _vp, _i]),
     "gs_loss_forward_batched": (_i, [_i, _i, _i, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
     "gs_loss_backward_batched": (_i, [_i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "gs_metrics_batched": (_i, [_i, _i, _i, _vp, _vp, _vp, _i, _vp, _vp]),
     "gs_profile_enable": (_i, [_i]),
     "gs_profile_read": (_i, [_i, C.POINTER(C.c_double), C.POINTER(_i64)]),
     "gs_profile_stage_name": (C.c_char_p, [_i]),

@@ -556,6 +556,44 @@ def fused_l1_ssim_batched(images, gts_u8, rows4):
     return _FusedL1SSIMBatched.apply(images, list(gts_u8), [tuple(int(v) for v in r) for r in rows4])
 
 
+def image_metrics_batched(images, gts_u8, rows4, saved=False):
+    """Held-out image metrics of B views in one launch (gs_metrics_batched); no autograd.
+    images (B,3,H,W) float32 CUDA; gts_u8: list of B CUDA uint8 windows (3, row1-row0, W) (None where row1 == row0);
+    rows4: B tuples (row0, row1, count_row0, count_row1), as for fused_l1_ssim_batched.  saved=False evaluates
+    clamp(image, 0, 1) (train_internal.py:471-478); saved=True the image after the 8-bit PNG round trip of
+    render.py:127-138 -> metrics.py:26-36.
+    -> (B,3,3) float64 on the device: [v][0][c] = sum |x-y|, [v][1][c] = sum (x-y)^2, [v][2][c] = sum ssim_map, over the
+    counted rows of channel c."""
+    if not isinstance(images, torch.Tensor) or images.dim() != 4 or images.shape[1] != 3:
+        raise ValueError(f"images must be a (B,3,H,W) tensor, got {getattr(images, 'shape', type(images))}")
+    images = _f32c(images, "images")
+    B, _, H, W = images.shape
+    gts_u8, rows4 = list(gts_u8), [tuple(int(v) for v in r) for r in rows4]
+    if not 1 <= B <= MAX_VIEWS:
+        raise ValueError(f"1..{MAX_VIEWS} views per call, got {B}")
+    if len(gts_u8) != B or len(rows4) != B or any(len(r) != 4 for r in rows4):
+        raise ValueError("one ground-truth window and one (row0,row1,count_row0,count_row1) per view")
+    keep = []
+    for k, (gt, (r0, r1, c0, c1)) in enumerate(zip(gts_u8, rows4)):
+        if not (0 <= r0 <= r1 <= H):
+            raise ValueError(f"view {k}: window rows [{r0},{r1}) outside [0,{H})")
+        if r1 == r0:
+            keep.append(None)
+            continue
+        if not (r0 <= c0 <= c1 <= r1):
+            raise ValueError(f"view {k}: counted rows [{c0},{c1}) must lie inside [{r0},{r1})")
+        if not isinstance(gt, torch.Tensor) or gt.dtype != torch.uint8 or not gt.is_cuda:
+            raise TypeError("gt windows must be CUDA uint8 tensors (3, rows, W)")
+        if tuple(gt.shape) != (3, r1 - r0, W):
+            raise ValueError(f"gt window {k} must be (3,{r1 - r0},{W}), got {tuple(gt.shape)}")
+        keep.append(gt.contiguous())
+    flat = _i32_array([v for r in rows4 for v in r])
+    gptr = (C.c_void_p * B)(*[None if g is None else g.data_ptr() for g in keep])
+    out = torch.empty((B, 3, 3), dtype=torch.float64, device=images.device)
+    _lib.call("gs_metrics_batched", B, H, W, flat, images.data_ptr(), gptr, 1 if saved else 0, out.data_ptr(), _stream())
+    return out
+
+
 def get_local2j_ids_bool(image_height, image_width, rank, world_size, means2D, radii, dist_global_strategy,
                          cuda_args=None):
     """(P, world_size) bool: does splat i touch rank j's flattened tile range.  `rank` is unused (kept for

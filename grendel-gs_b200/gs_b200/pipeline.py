@@ -40,7 +40,8 @@ class DeviceCamera:
         self.viewmatrix = torch.as_tensor(cam["viewmatrix"], dtype=torch.float32).to(device)
         self.projmatrix = torch.as_tensor(cam["projmatrix"], dtype=torch.float32).to(device)
         self.campos = torch.as_tensor(cam["campos"], dtype=torch.float32).to(device)
-        self.bg = torch.tensor(bg, dtype=torch.float32, device=device)
+        self.bg_host = tuple(float(v) for v in bg)
+        self.bg = torch.tensor(self.bg_host, dtype=torch.float32, device=device)
 
     def settings(self, sh_degree=None):
         return RasterSettings(image_height=self.image_height, image_width=self.image_width, tanfovx=self.tanfovx,
@@ -498,6 +499,20 @@ class Trainer:
         dist.all_gather_into_tensor(allt, loc, group=self.group)
         times = allt.reshape(self.world, B).cpu().tolist()       # gpu_camera_running_time[gpu][camera]
         finish_strategy(self.history, strategies, times, self.iteration, self.world, self.H, self.W, self.heuristic_decay)
+
+    def evaluate(self, cams, gts, batch_size=None, protocol="report"):
+        """Render held-out views with the current parameters and compare them with their ground truth (forward only; no
+        effect on training state: division history, iteration, pending timing feedback, gradients, means2D / radii of
+        the last step and last_info() stay as they were).
+        cams: camera dicts (synthetic.make_camera) or DeviceCamera, all of one image size and background; gts: one uint8
+        (3,H,W) tensor per camera, host or device (with distributed_dataset_storage only rank 0 holds them: pass None
+        elsewhere).  Views go through in batches of batch_size (default: the training batch size), each split into
+        uniform tile-row strips over the ranks.  Every rank must call it with the same cameras.
+        protocol: "report" = training_report's numbers (train_internal.py:466-479: clamped image, PSNR averaged over
+        channels); "saved" = render.py + metrics.py's (the image quantised to 8 bits as saved to PNG, one PSNR over the
+        image).  -> {"per_view": [{"uid", "l1", "psnr", "ssim"}, ...], "l1", "psnr", "ssim"} (means over the views)."""
+        from . import evaluate as _ev
+        return _ev.run(self, cams, gts, batch_size, protocol)
 
     GROUP_OF = {"xyz": "_xyz", "f_dc": "_features_dc", "f_rest": "_features_rest", "opacity": "_opacity",
                 "scaling": "_scaling", "rotation": "_rotation"}

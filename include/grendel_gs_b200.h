@@ -313,6 +313,20 @@ GS_API int gs_loss_backward_batched(int num_views, int image_height, int image_w
                                     const float *image, const void *const *gt_u8_ptrs_host, const void *temp,
                                     const float *grad_l1, const float *grad_ssim, float *dL_dimage, void *stream);
 
+/* ---- held-out evaluation -- train_internal.py:466-479, render.py:120-138 -> metrics.py:26-36 ----------------
+ * Forward-only image metrics of B views in one launch: the loss forward's 11x11 window without derivative maps.  Per
+ * view v and channel c, over the counted rows [count_row0, count_row1) of the window [row0, row1) (rows4_host as in
+ * gs_loss_forward_batched; row1 == row0: the view's sums are 0), out_sums (B,3,3) fp64 is OVERWRITTEN with
+ *   out_sums[v][0][c] = sum |x - y|,  out_sums[v][1][c] = sum (x - y)^2,  out_sums[v][2][c] = sum ssim_map(x, y)
+ * where y = gt_u8 / 255 and x = clamp(image, 0, 1) (saved_mode 0: training_report, utils/image_utils.py:19-21) or,
+ * saved_mode 1, that value after torchvision.utils.save_image's 8-bit quantisation and to_tensor's read-back,
+ * uint8(min(255, x * 255 + 0.5)) / 255 with the multiply and add rounded separately (render.py:127-138).
+ * images: (B,3,H,W); gt_u8_host_array: HOST array of B device pointers to the (3, row1-row0, W) uint8 windows.
+ * Every per-pixel term is added in fp64: a view split into strips with 5-row halos sums to its whole-image value. */
+GS_API int gs_metrics_batched(int num_views, int image_height, int image_width, const int32_t *rows4_host,
+                              const float *images, const uint8_t *const *gt_u8_host_array, int saved_mode,
+                              double *out_sums, void *stream);
+
 /* ---- all-to-all staging -- gaussian_renderer/__init__.py:590-607,651-658 --------------------------
  * Replaces the per-(destination, camera) nonzero() + index_select + torch.cat glue around the sparse
  * all-to-all: rows of 11 floats forward (means2D 2, rgb 3, conic_opacity 4, radius as float, depth), 9 floats
